@@ -16,12 +16,16 @@ over the 10 M records, so that the default 16 timed steps are about one second o
            handle on ONE thread (tfr_decode_submit + tfr_batch_to_host_async keep H2D / kernels / D2H overlapped).
   roofline: the dominant kernel (decode_tile_kernel: the whole decode in one pass -- reads the framed input once, writes
            every Arrow byte once): algorithmic bytes per launch / its mean launch time (CUDA events recorded by the library
-           around every launch in the timed region), against the measured HBM copy bandwidth in MEASURED_PEAKS.json.
+           around every launch in the timed region), against the HBM copy bandwidth this run measures on the same GPU.
   parity_checked: after the timed loop one pool batch is decoded again in the very mode that was timed and compared, bit
            for bit and over all of its records, with the CPU oracle.
   cpu_baseline: the oracle port (C restatement of the reference's per-record algorithm) on the host cores.
   extra  : side metrics, each with its own roofline: configs[2] encode, configs[3] SequenceExample decode, configs[1]
            with ragged bytes columns, ByteArray records.
+
+  --dump-outputs DIR: after the timed steps, the columns the last decode of the last timed step returned are written to
+           DIR as float .npy files (see dump_outputs), so that two builds can be compared output for output: with the same
+           arguments the inputs are the same seeded records in every run.
 
 The synthetic columns are seeded numpy data; our arm frames them with the product's GPU encoder (proved byte-identical
 to the reference writer by tests/test_gpu_encode.py and tests/test_gpu_scale.py), the CPU arm with the oracle's writer.
@@ -36,6 +40,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 from concurrent.futures import ThreadPoolExecutor
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -65,7 +70,11 @@ def parse_args():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed decode returned to DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.dump_outputs is not None and (args.impl != "ours" or args.steps < 1):
+        ap.error("--dump-outputs writes the last timed step of the GPU arm: it needs --impl ours and --steps >= 1")
+    return args
 
 
 def dist_env():
@@ -469,6 +478,79 @@ def parity_check(dec, schema, d_batch, h_batch, threads):
 
 
 # ---------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path returned, as float .npy files
+# ---------------------------------------------------------------------------------------------
+DUMP_ROWS = 8192            # rows of the seeded sample written value by value
+DUMP_SEED = 7
+DUMP_LIMIT = 64 << 20       # bytes of all files together
+
+
+def _exact_float(a: np.ndarray) -> np.ndarray:
+    """`a` as float32 / float64 without rounding: floats stay, bytes and int32 widen exactly, and an int64 becomes two
+    float64 columns (signed high word, unsigned low word)"""
+    if a.dtype in (np.float32, np.float64):
+        return a
+    if a.dtype == np.uint8:
+        return a.astype(np.float32)
+    if a.dtype == np.int32:
+        return a.astype(np.float64)
+    if a.dtype == np.int64:
+        return np.stack([(a >> 32).astype(np.float64), (a & 0xFFFFFFFF).astype(np.float64)], axis=1)
+    raise TypeError(f"no exact float form for {a.dtype}")
+
+
+def dump_outputs(out_dir, names, cols):
+    """Writes the host copy of a decoded batch to out_dir and returns the bytes written:
+      digest.npy        per column: n_rows, null_count, CRC-32 of its validity bits, of its offsets and of its values (over
+                        every row), number of values
+      rows.npy          a fixed, seeded sample of row indices
+      valid.npy         validity (0/1) of the sampled rows, one row per column
+      <name>.npy        the values of the sampled rows, in row order (int64 as [high word, low word] pairs)
+      <name>.lengths.npy  for list and bytes columns: the number of values of each sampled row"""
+    os.makedirs(out_dir, exist_ok=True)
+    n = cols[0].n_rows if cols else 0
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_ROWS), replace=False))
+    arrays = {"rows": rows.astype(np.float64)}
+    digest, valid = [], []
+    for name, c in zip(names, cols):
+        bits = np.ones(n, np.uint8) if c.validity is None else np.unpackbits(c.validity, bitorder="little")[:n]
+        digest.append([c.n_rows, c.null_count, zlib.crc32(np.packbits(bits, bitorder="little").tobytes()),
+                       zlib.crc32(b"".join(o.tobytes() for o in c.offsets)), zlib.crc32(c.values.tobytes()), len(c.values)])
+        valid.append(bits[rows].astype(np.float32))
+        lo, hi = rows, rows + 1
+        for o in c.offsets:                 # a row's children are one contiguous range at every level
+            lo, hi = o[lo].astype(np.int64), o[hi].astype(np.int64)
+        lens = hi - lo
+        if c.offsets:
+            arrays[f"{name}.lengths"] = lens.astype(np.float64)
+        idx = np.repeat(lo - (np.cumsum(lens) - lens), lens) + np.arange(int(lens.sum()))
+        arrays[name] = _exact_float(c.values[idx])
+    arrays["valid"] = np.array(valid, dtype=np.float32)
+    arrays["digest"] = np.array(digest, dtype=np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, f"--dump-outputs would write {total} bytes (limit {DUMP_LIMIT})"
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+    return total
+
+
+def hbm_copy_gbs(torch, dev, reps=10):
+    """HBM bandwidth as a device-to-device copy reaches it (bytes read + bytes written): 1 Gi bf16 elements, best of `reps`"""
+    a = torch.empty(1 << 30, dtype=torch.bfloat16, device=dev)
+    b = torch.empty_like(a)
+    b.copy_(a)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    best = float("inf")
+    for _ in range(reps):
+        e0.record()
+        b.copy_(a)
+        e1.record()
+        e1.synchronize()
+        best = min(best, e0.elapsed_time(e1))
+    return 2 * a.nbytes / (best * 1e-3) / 1e9
+
+
+# ---------------------------------------------------------------------------------------------
 # side metrics (rank 0, N = 1): each a short resident loop with its own roofline
 # ---------------------------------------------------------------------------------------------
 def _roof(alg_bytes, ms, peak):
@@ -727,18 +809,24 @@ def run_ours(args):
         out_bytes = b.info["out_bytes"]
         b.release()
 
-    def resident_steps(steps, k0=0):
+    def resident_steps(steps, k0=0, keep_last=False):
+        """`steps` x --batches-per-step pipelined decodes; keep_last: the last batch is returned unreleased"""
         nb = 0
         k = k0
+        b = None
         for _ in range(steps):
             for _ in range(args.batches_per_step):
+                if b is not None:
+                    b.release()               # the work stays enqueued; the lane is recycled when its kernels are done
                 b = dec.submit(d_batches[k % P])
-                b.release()                   # the work stays enqueued; the lane is recycled when its kernels are done
                 nb += batch_bytes[k % P]
                 k += 1
-        return nb, k
+        if b is not None and not keep_last:
+            b.release()
+            b = None
+        return nb, k, b
 
-    _, k = resident_steps(args.warmup)
+    _, k, _ = resident_steps(args.warmup)
     torch.cuda.synchronize()
     stats0 = dec.stats()
     dec.set_profiling(True)
@@ -748,7 +836,7 @@ def run_ours(args):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_wall0 = time.perf_counter()
     ev0.record(stream)
-    in_bytes, k = resident_steps(args.steps, k)
+    in_bytes, k, last = resident_steps(args.steps, k, keep_last=args.dump_outputs is not None and rank == 0)
     ev1.record(stream)
     barrier()
     t_wall = time.perf_counter() - t_wall0
@@ -760,6 +848,16 @@ def run_ours(args):
     timed_stats = {k2: stats1[k2] - stats0[k2] for k2 in stats1}
     # every timed decode ran in the pipelined single-pass mode and none was flagged (a flagged batch would have been redone)
     assert timed_stats["speculative_submits"] == n_timed and timed_stats["speculative_redone"] == 0, timed_stats
+
+    # ---------------- --dump-outputs: the columns the last timed decode returned ----------------
+    dumped = None
+    if last is not None:
+        cols = last.to_host()
+        assert last.info["error_code"] == 0, last.info
+        dumped = {"dir": args.dump_outputs, "pool_batch": (k - 1) % P, "rows": int(last.n_rows),
+                  "sampled_rows": min(int(last.n_rows), DUMP_ROWS), "bytes": dump_outputs(args.dump_outputs, schema.names, cols)}
+        last.release()
+        del cols
 
     # ---------------- parity of the timed mode, whole batch ----------------
     parity = None
@@ -892,14 +990,8 @@ def run_ours(args):
 
     value = tot_in / (ms * 1e-3) / 1e9
     # ---------------- roofline of the dominant kernel ----------------
-    peaks = {}
-    try:
-        with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
-            peaks = json.load(f)
-    except Exception:
-        pass
-    peak = float(peaks.get("hbm_gbs", 6650.0))
-    peak_src = "measured (MEASURED_PEAKS.json hbm_gbs)" if "hbm_gbs" in peaks else "fallback 6650 GB/s (B200_PROFILING.md)"
+    peak = hbm_copy_gbs(torch, dev)
+    peak_src = "measured by this run on the same GPU: device copy of 1 Gi bf16 elements (bytes read + written), best of 10"
     p1_alg = batch_bytes[0] + int(out_bytes)        # framed input read once + Arrow output written once (algorithmic bytes of the whole decode of one batch)
     p1_ms = prof["ms"]["pass1"] / max(1, prof["pass1_launches"])
     achieved = p1_alg / (p1_ms * 1e-3) / 1e9 if p1_ms > 0 else 0.0
@@ -940,6 +1032,8 @@ def run_ours(args):
     }
     if parity:
         line["parity_checked"] = parity
+    if dumped:
+        line["dumped_outputs"] = dumped
     if infer:
         line["schema_inference_reduce"] = infer
     if cfg5:
