@@ -129,7 +129,8 @@ int32_t tfr_decoder_num_staging_slots(void);
  *                 The buffer must stay valid and unchanged until the batch has been waited on.
  *   is_final    : nonzero -> a trailing partial record is TFR_E_TRUNCATED (EOF inside a
  *                 record); zero -> it is left unconsumed (see *consumed).
- * tfr_decode returns when the batch is complete and verified (*consumed is final).
+ * tfr_decode returns when the batch is complete and verified (*consumed is final): no kernel
+ * reads `data` any more, so a device buffer may be overwritten or freed right away.
  * A data error does not fail the call: rows before the first bad record are delivered and
  * the error is reported by tfr_batch_status, like the reference's iterator which yields
  * rows until the throwing record.
@@ -232,7 +233,15 @@ void    tfr_encoder_destroy(tfr_encoder*);
  * fields.  Produces the framed bytes of all rows, in row order, byte-identical to what the
  * reference writer appends to its output stream.  *out_dev is device memory owned by the
  * encoder, valid until the next tfr_encode/destroy.  A null in a non-nullable column is
- * TFR_E_NULL_IN_NONNULL with *error_row set.                                               */
+ * TFR_E_NULL_IN_NONNULL with *error_row set.
+ * tfr_encode may return with the last kernel still queued on tfr_encoder_stream:
+ *   - host columns (columns_on_device == 0) have been copied when the call returns and may
+ *     be reused or freed at once;
+ *   - device columns are read by that kernel: keep them valid and unchanged until the
+ *     encoder's stream has drained (tfr_encoder_result_host returns, the stream is
+ *     synchronised, or the caller's own work is ordered behind it with an event);
+ *   - *out_dev holds the bytes once the same point is reached: device consumers order their
+ *     reads behind tfr_encoder_stream; tfr_encoder_result_host waits itself.               */
 int32_t tfr_encode(tfr_encoder*, const tfr_column* columns, int32_t n, int32_t columns_on_device,
                    void** out_dev, size_t* out_bytes, int64_t* error_row);
 /* copy the last encode result to host memory (pinned staging owned by the encoder) */

@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <memory>
 #include <mutex>
 #include <string>
@@ -83,8 +84,23 @@ struct DeviceCtx {
   cudaError_t err = cudaSuccess;
   int sm_count = 148;
   int max_smem_optin = 48 * 1024;
+  std::mutex smem_mu;                                  // guards smem_set
+  std::map<const void*, size_t> smem_set;              // kernel -> the opt-in dynamic shared memory set on this device
 };
 static DeviceCtx g_ctx[64];
+
+// The opt-in limit of dynamic shared memory is an attribute of the kernel on the device, shared by every handle and thread,
+// and cudaFuncSetAttribute SETS it.  This is its one owner: the value only ever grows, and it is read, compared and set under
+// the device's lock, so a launch with at most `bytes` is valid afterwards whatever other handles launch meanwhile.  The
+// caller has made ctx's device current.
+static cudaError_t ensure_dyn_smem(DeviceCtx* ctx, const void* kernel, size_t bytes) {
+  std::lock_guard<std::mutex> lk(ctx->smem_mu);
+  size_t& cur = ctx->smem_set[kernel];
+  if (cur >= bytes) return cudaSuccess;
+  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  if (e == cudaSuccess) cur = bytes;
+  return e;
+}
 
 static void build_crc_tables(CrcTables& t) {
   const uint32_t POLY = 0x82F63B78u;
